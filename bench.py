@@ -332,6 +332,8 @@ def run_reference(args):
     for _ in range(args.steps):
         val = cpu_eval(name, hp, threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"objective": np.array([val], dtype=np.float64)})
     v = args.steps / dt
     line = {
         "impl": "reference", "metric": "objective_evals_per_sec", "value": v, "unit": "evals/s", "n_gpus": args.gpus,
@@ -509,6 +511,8 @@ def run_ours(args):
     lib.gpk_launch_count_reset()
     ms_total, per_step = timed_loop(torch, dist, steps, lambda i: arm.eval_resident(), slots)
     launches = int(lib.gpk_launch_count())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"objective": slots[-1:].cpu().numpy()})
     objective = float(slots[-1].item()) / world
     ms_total, table = gather_ms(torch, dist, world, ms_total, per_step)
     ms_step = ms_total / steps
@@ -753,6 +757,14 @@ def run_ours(args):
 _REAL_STDOUT = None
 
 
+def dump_outputs(out_dir: str, arrays: dict):
+    """Writes what the timed path returned in its last step as out_dir/<name>.npy (float64). The inputs are seeded,
+    so two builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def emit(line: dict):
     """The ONE JSON line of the contract, on the process's original stdout."""
     out = _REAL_STDOUT if _REAL_STDOUT is not None else sys.stdout
@@ -774,7 +786,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="gpr_c2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-svgp", action="store_true", help="skip the SVGP C4 sharding-mode section")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the objective of the last timed step as DIR/objective.npy (float64, shape [1]; "
+                         "summed over ranks under torchrun)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -190,6 +190,22 @@ def test_bench_reference_arm_prints_one_json_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["higher_is_better"] is True
 
 
+def test_bench_dump_outputs_writes_the_last_step_objective(tmp_path):
+    """--dump-outputs DIR: the objective of the last timed step as DIR/objective.npy, the value the JSON line reports."""
+    import json
+    import subprocess
+    import sys
+
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "gpr_c1",
+                        "--steps", "1", "--warmup", "0", "--dump-outputs", str(tmp_path / "out")],
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads(r.stdout.strip())
+    got = np.load(tmp_path / "out" / "objective.npy")
+    assert got.dtype == np.float64 and got.shape == (1,)
+    assert got[0] == d["objective"] and d["steps"] == 1
+
+
 def test_kernel_expressions_pass_the_host_compile_path_without_gpu():
     """Every leaf op (incl. Polynomial, whose offset / degree ride in the lengthscale / alpha fields) must get past the
     C-ABI's argument and expression checks (status -1 -> ValueError); without a device the call then fails only at
