@@ -110,6 +110,10 @@ SIGNATURES = {
     "gpk_sgpr_elbo": (c_int, [_KN, c_int, _I32, _F64, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64,
                               c_void_p, c_int64, c_int64, c_double, c_double, c_int, c_void_p, c_void_p, c_void_p,
                               c_void_p, c_void_p, c_void_p]),
+    "gpk_sgpr_elbo_grad_ws": (c_size_t, [c_int64, c_int64, c_int64, c_int]),
+    "gpk_sgpr_elbo_grad": (c_int, [_KN, c_int, _I32, _F64, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64,
+                                   c_void_p, c_int64, c_int64, c_double, c_double, c_int, c_void_p, c_int, c_void_p,
+                                   c_int64, c_void_p, c_void_p]),
     "gpk_svgp_elbo_ws": (c_size_t, [c_int64, c_int64, c_int64, c_int]),
     "gpk_svgp_elbo": (c_int, [_KN, c_int, _I32, _F64, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64,
                               c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int, c_int, c_double, c_double,

@@ -92,6 +92,10 @@ size_t sgpr_elbo_ws(int64_t N, int64_t M, int64_t P, int dtype);
 int sgpr_elbo(const gpk_knode*, int, const int32_t*, const double*, const void*, int64_t, int64_t, int64_t, const void*,
               int64_t, const void*, int64_t, int64_t, double, double, int, double*, void*, void*, void*, void*,
               cudaStream_t);
+size_t sgpr_elbo_grad_ws(int64_t N, int64_t M, int64_t P, int dtype);
+int sgpr_elbo_grad(const gpk_knode*, int, const int32_t*, const double*, const void*, int64_t, int64_t, int64_t,
+                   const void*, int64_t, const void*, int64_t, int64_t, double, double, int, double*, int, double*,
+                   int64_t, void*, cudaStream_t);
 size_t svgp_elbo_ws(int64_t B, int64_t M, int64_t P, int dtype);
 int svgp_elbo(const gpk_knode*, int, const int32_t*, const double*, const void*, int64_t, int64_t, int64_t, const void*,
               int64_t, const void*, int64_t, int64_t, const void*, const void*, int, int, double, double, double, int,
@@ -360,6 +364,17 @@ int gpk_gpr_lml_grad(const gpk_knode* nodes, int n_nodes, const int32_t* dims, c
   GPK_DTYPE_OK("gpr_lml_grad");
   return gpr_lml_grad(nodes, n_nodes, dims, ard, X, N, ldx, D, Yc, P, noise_variance, dtype, out, n_out, ws,
                       (cudaStream_t)stream);
+}
+
+size_t gpk_sgpr_elbo_grad_ws(int64_t N, int64_t M, int64_t P, int dtype) { return sgpr_elbo_grad_ws(N, M, P, dtype); }
+
+int gpk_sgpr_elbo_grad(const gpk_knode* nodes, int n_nodes, const int32_t* dims, const double* ard, const void* X,
+                       int64_t N, int64_t ldx, int64_t D, const void* Yc, int64_t P, const void* Z, int64_t M,
+                       int64_t ldz, double noise_variance, double jitter, int dtype, double* out, int n_out, double* dZ,
+                       int64_t lddz, void* ws, void* stream) {
+  GPK_DTYPE_OK("sgpr_elbo_grad");
+  return sgpr_elbo_grad(nodes, n_nodes, dims, ard, X, N, ldx, D, Yc, P, Z, M, ldz, noise_variance, jitter, dtype, out,
+                        n_out, dZ, lddz, ws, (cudaStream_t)stream);
 }
 
 size_t gpk_svgp_elbo_A(int64_t B, int64_t M, int64_t P, int dtype, int64_t* ld) { return svgp_elbo_A(B, M, P, dtype, ld); }

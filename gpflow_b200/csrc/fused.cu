@@ -240,6 +240,62 @@ int sgpr_elbo(const gpk_knode* nodes, int n_nodes, const int32_t* dims, const do
   return 0;
 }
 
+// ---- value + gradient (grad.cu) -----------------------------------------------------------------
+int sgpr_grad_check(const gpk_knode* nodes, int n_nodes, const int32_t* dims, const double* ard, int64_t D);
+int sgpr_grad_backward(const gpk_knode* nodes, int n_nodes, const int32_t* dims, const double* ard, const void* X,
+                       int64_t N, int64_t ldx, int64_t D, const void* Yc, int64_t P, const void* Z, int64_t M,
+                       int64_t ldz, double noise, int dtype, const void* L, const void* LB, int64_t ldm, const void* Ap,
+                       int64_t ldn, const void* c, const double* scal, const SgprBwdWs& b, double* out, int n_out,
+                       double* dZ, int64_t lddz, cudaStream_t st);
+
+struct SgprGradWs {
+  SgprWs f; SgprBwdWs b; size_t bytes;
+};
+static SgprGradWs sgpr_grad_layout(void* ws, int64_t N, int64_t M, int64_t P, int dtype) {
+  SgprGradWs w;
+  w.f = sgpr_layout(ws, N, M, P, dtype);
+  Arena a(ws);
+  a.off = w.f.bytes;
+  const size_t ts = dtype_size(dtype), mm = (size_t)M * w.f.ldm * sizeof(double);
+  const int64_t h = M / 2 + NB;
+  SgprBwdWs& b = w.b;
+  double** sq[] = {&b.Li, &b.LBi, &b.B, &b.Bi, &b.C, &b.H, &b.G1, &b.T, &b.dKuu};
+  for (double** p : sq) *p = (double*)a.take(mm);
+  b.dinvL = (double*)a.take(dinv_bytes(M, GPK_F64));
+  b.dinvB = (double*)a.take(dinv_bytes(M, GPK_F64));
+  b.tmp = (double*)a.take((size_t)h * h * sizeof(double));
+  b.cw = (double*)a.take((size_t)M * P * sizeof(double));
+  b.wt = (double*)a.take((size_t)M * P * sizeof(double));
+  b.v = (double*)a.take((size_t)M * P * sizeof(double));
+  b.sc = (double*)a.take(256);
+  b.G1n = dtype == GPK_F32 ? a.take((size_t)M * w.f.ldm * ts) : nullptr;
+  b.dKuf = a.take((size_t)M * w.f.ldn * ts);
+  w.bytes = a.off;
+  return w;
+}
+
+size_t sgpr_elbo_grad_ws(int64_t N, int64_t M, int64_t P, int dtype) {
+  return sgpr_grad_layout(nullptr, N, M, P, dtype).bytes;
+}
+
+// out: [0..7] as sgpr_elbo; [8] d/dvariance, [9] d/dnoise_variance, [10 ...] d/dlengthscale (1 or n_ard entries);
+// dZ [M, D] (lddz) fp64
+int sgpr_elbo_grad(const gpk_knode* nodes, int n_nodes, const int32_t* dims, const double* ard, const void* X, int64_t N,
+                   int64_t ldx, int64_t D, const void* Yc, int64_t P, const void* Z, int64_t M, int64_t ldz,
+                   double noise, double jitter, int dtype, double* out, int n_out, double* dZ, int64_t lddz, void* ws,
+                   cudaStream_t st) {
+  GPK_CHECK_ARG(N > 0 && M > 0 && P > 0 && D > 0 && ws && out && Yc && dZ && lddz >= D, "sgpr_elbo_grad: bad arguments");
+  GPK_TRY(sgpr_grad_check(nodes, n_nodes, dims, ard, D));
+  const int n_l = nodes[0].n_ard > 0 ? nodes[0].n_ard : 1;
+  GPK_CHECK_ARG(n_out >= 10 + n_l, "sgpr_elbo_grad: n_out = %d < %d", n_out, 10 + n_l);
+  SgprGradWs w = sgpr_grad_layout(ws, N, M, P, dtype);
+  // forward pass (sgpr.py:181-289) into the head of the workspace: L, A' = L^-1 Kuf, LB, c and the scalars stay there
+  GPK_TRY(sgpr_elbo(nodes, n_nodes, dims, ard, X, N, ldx, D, Yc, P, Z, M, ldz, noise, jitter, dtype, out, nullptr,
+                    nullptr, nullptr, ws, st));
+  return sgpr_grad_backward(nodes, n_nodes, dims, ard, X, N, ldx, D, Yc, P, Z, M, ldz, noise, dtype, w.f.Kuu, w.f.Bm,
+                            w.f.ldm, w.f.Kuf, w.f.ldn, w.f.c, w.f.scal, w.b, out, n_out, dZ, lddz, st);
+}
+
 // ---------------------------------------------------------------------------------------------
 // SVGP
 // ---------------------------------------------------------------------------------------------

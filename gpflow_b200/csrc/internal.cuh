@@ -45,6 +45,14 @@ int trsm_any(int trans, const void* L, int64_t n, int64_t ldl, void* B, int64_t 
              const void* dinv, cudaStream_t st);
 int trtri_diag_any(const void* L, int64_t n, int64_t ldl, void* dinv, int dtype, cudaStream_t st);
 
+// Scratch of the SGPR ELBO backward (grad.cu), laid out by fused.cu behind the forward's workspace.  fp64 [M, ldm]:
+// Li, LBi (the factors, inverted in place), B, Bi, C, H, G1, T, dKuu; fp64 [M, P]: cw, wt, v; dinvL / dinvB: 128-block
+// inverses; tmp: (M/2 + 128)^2 doubles; sc: 2 scalars; G1n: G1 in the model dtype; dKuf: [M, ldn] model dtype.
+struct SgprBwdWs {
+  double *Li, *LBi, *B, *Bi, *C, *H, *G1, *T, *dKuu, *dinvL, *dinvB, *tmp, *cw, *wt, *v, *sc;
+  void *G1n, *dKuf;
+};
+
 inline size_t dinv_bytes(int64_t n, int dtype) { return (size_t)((n + NB - 1) / NB) * NB * NB * dtype_size(dtype); }
 inline size_t potrf_ws_bytes(int64_t n, int64_t rows, int dtype) {
   return align_up(dinv_bytes(n, dtype), 256) + 256 /* look-ahead counter */ + potrf_tc_ws_bytes(n, rows, dtype);

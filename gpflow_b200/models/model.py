@@ -99,7 +99,8 @@ class LossClosure:
 
     def __init__(self, model, loss_fn: Callable[[], Any]):
         self._model, self._loss_fn = model, loss_fn
-        if hasattr(model, "training_loss_and_gradients"):
+        # a subclass that optimises another objective sets the attribute to None (GPRFITC under SGPR)
+        if getattr(model, "training_loss_and_gradients", None) is not None:
             self.value_and_gradients = self._value_and_gradients
 
     def __call__(self):

@@ -3,6 +3,8 @@ from __future__ import annotations
 
 from typing import Any, NamedTuple, Optional, Tuple
 
+import numpy as np
+
 from .. import _lib, config, covariances, ops, posteriors
 from ..inducing_variables import InducingPoints, inducingpoint_wrapper
 from ..kernels import Kernel, compile_kernel
@@ -76,6 +78,69 @@ class SGPR(GPModel, InternalDataTrainingLossMixin):
         self._last = _sgpr_fused(X, Y, self.kernel, self.inducing_variable, self.likelihood, self.mean_function,
                                  owner=self)
         return ops.objective(self._last, 0, 7)
+
+    def elbo_and_grad(self):
+        """Value and gradient in ONE fused call (gpk_sgpr_elbo_grad): the backward pass the reference gets from TensorFlow
+        autodiff through sgpr.py:181-289.  Returns (elbo, grads): `elbo` as elbo(); `grads` a dict
+        {Parameter: dELBO/d(constrained value)} for the kernel variance, the lengthscale(s), the likelihood variance and
+        the inducing points Z ([M, D], zero outside the kernel's active dims), NumPy after one device->host read.
+        Covers a single stationary leaf kernel, a constant Gaussian noise variance and InducingPoints, float32 / float64."""
+        from ..kernels.stationaries import Stationary
+
+        k = self.kernel
+        if not isinstance(k, Stationary) or k._op not in (_lib.K_RBF, _lib.K_MATERN12, _lib.K_MATERN32,
+                                                          _lib.K_MATERN52, _lib.K_EXPONENTIAL):
+            raise NotImplementedError("the device backward pass covers a single SquaredExponential / Matern12 / "
+                                      "Matern32 / Matern52 / Exponential kernel")
+        if self.likelihood.heteroskedastic or self.likelihood.variance is None:
+            raise NotImplementedError("the device backward pass covers Gaussian(variance=...)")
+        iv = self.inducing_variable
+        if not isinstance(iv, InducingPoints):
+            raise NotImplementedError("the device backward pass covers InducingPoints")
+        lib = _lib.load()
+        X, Y = self.data
+        N, D = X.shape
+        P = Y.shape[1]
+        Z = ops.to_device(iv.Z)
+        M = Z.shape[0]
+        dc = ops.dtype_code(X)
+        need = lib.gpk_sgpr_elbo_grad_ws(N, M, P, dc)
+        if getattr(self, "_sgpr_gws", None) is None or self._sgpr_gws.numel() < need or self._sgpr_gws.device != X.device:
+            self._sgpr_gws = ops.scratch_bytes(need)
+        nl = int(k.lengthscales.numpy().size) if k.ard else 1
+        n_out = 10 + nl
+        # one fp64 buffer holds the scalars and dZ [M, D], so the host reads both in one transfer
+        buf = ops.torch().empty((n_out + M * D,), dtype=ops.torch().float64, device=X.device)
+        out, dZ = buf[:n_out], buf[n_out:]
+        if isinstance(self.mean_function, Zero):
+            Yc = Y
+        else:
+            Yc = ops.axpby(-1.0, self.mean_function(X), 1.0, ops.copy(Y))
+        nodes, n_nodes, dims, ard = compile_kernel(k, D)
+        _lib.check(lib.gpk_sgpr_elbo_grad(nodes, n_nodes, dims, ard, ops._p(X), N, ops._ld(X), D, ops._p(Yc), P,
+                                          ops._p(Z), M, ops._ld(Z), self.likelihood._variance_value(),
+                                          config.default_jitter(), dc, ops._p(out), n_out, ops._p(dZ), D,
+                                          ops._p(self._sgpr_gws), ops._stream()), "gpk_sgpr_elbo_grad")
+        self._last = out
+        h = buf.cpu().numpy()
+        if int(h[7]) != 0:
+            raise ops.NonPositiveDefiniteError(f"Cholesky decomposition was not successful (pivot {int(h[7])} <= 0)")
+        grads = {k.variance: np.asarray(h[8]), self.likelihood.variance: np.asarray(h[9]),
+                 k.lengthscales: (h[10:10 + nl].copy() if k.ard else np.asarray(h[10])),
+                 iv.Z: h[n_out:].reshape(M, D).copy()}
+        return ops.objective(out, 0, 7), grads
+
+    def training_loss_and_gradients(self):
+        """(loss, gradients) for the optimiser contract of gpflow/optimizers/scipy.py:322-331: loss = -ELBO (float) and
+        one gradient per TRAINABLE parameter w.r.t. its UNCONSTRAINED variable, in `trainable_parameters` order."""
+        elbo, grads = self.elbo_and_grad()
+        out = []
+        for p in self.trainable_parameters:
+            if p not in grads:
+                raise NotImplementedError("a trainable parameter has no device gradient (mean-function parameters, "
+                                          "priors and data gradients are outside the hot path)")
+            out.append(-p.unconstrained_gradient(grads[p]))
+        return -float(elbo), out
 
     def elbo_terms(self):
         """(const, logdet_term, quad_term) of the last evaluation as device scalars (sgpr.py:214-271)."""
@@ -202,7 +267,14 @@ class GPRFITC(SGPR):
     def maximum_log_likelihood_objective(self):  # sgpr.py:434-435
         return self.fitc_log_marginal_likelihood()
 
+    # GPRFITC optimises fitc_log_marginal_likelihood(), which has no device backward pass: its training closure offers
+    # no value_and_gradients
+    training_loss_and_gradients = None
+
     def elbo(self):
+        raise NotImplementedError("GPRFITC optimises fitc_log_marginal_likelihood(), not an ELBO")
+
+    def elbo_and_grad(self):
         raise NotImplementedError("GPRFITC optimises fitc_log_marginal_likelihood(), not an ELBO")
 
     def fitc_log_marginal_likelihood(self):

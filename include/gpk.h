@@ -271,6 +271,25 @@ GPK_API int gpk_sgpr_elbo(const gpk_knode* nodes, int n_nodes, const int32_t* di
                   int dtype, double* out, void* cache_L, void* cache_LB, void* cache_c, void* ws,
                   void* stream);
 
+/* SGPR ELBO AND its gradient w.r.t. the kernel variance, the likelihood variance, the lengthscale(s) and the inducing
+ * points: the backward pass that TensorFlow autodiff supplies to the reference's optimiser (gpflow/optimizers/scipy.py:78-228
+ * -> models/training_mixins.py:43-78 -> models/sgpr.py:181-289), written out (DESIGN.md section 4.9).  The forward of
+ * gpk_sgpr_elbo runs unchanged into the head of the workspace; the backward then forms, in fp64, L^-1, LB^-1, B^-1 and
+ * dELBO/dKuu, computes dELBO/dKuf = (L^-T C A' + v E^T) / s2 with one M x M x N GEMM in the model dtype, and reduces
+ * dK (.) dK/dtheta over the Kuf and Kuu tiles.  No host synchronisation.  Covers a single stationary leaf kernel (RBF,
+ * Matern12/32/52, Exponential; scalar or ARD lengthscale; active_dims), float32 and float64.  Arguments as gpk_sgpr_elbo
+ * without the cache pointers, plus:
+ *   out: device double[n_out]: [0..7] as gpk_sgpr_elbo, [8] d/dvariance, [9] d/dnoise_variance,
+ *        [10 .. 10 + n_l) d/dlengthscale (n_l = 1, or the number of ARD lengthscales); n_out >= 10 + n_l.
+ *   dZ:  device double [M, D] (lddz >= D): d/dZ; zero in the columns outside the kernel's active dims.
+ *   ws:  gpk_sgpr_elbo_grad_ws(N, M, P, dtype) bytes. */
+GPK_API size_t gpk_sgpr_elbo_grad_ws(int64_t N, int64_t M, int64_t P, int dtype);
+GPK_API int gpk_sgpr_elbo_grad(const gpk_knode* nodes, int n_nodes, const int32_t* dims, const double* ard,
+                       const void* X, int64_t N, int64_t ldx, int64_t D, const void* Yc, int64_t P,
+                       const void* Z, int64_t M, int64_t ldz, double noise_variance, double jitter,
+                       int dtype, double* out, int n_out, double* dZ, int64_t lddz, void* ws,
+                       void* stream);
+
 /* SVGP.elbo (gpflow/models/svgp.py:166-181) for a single-output kernel shared by P latent GPs
  * (posteriors.py:827-841 -> conditionals/util.py:84-169 -> kullback_leiblers.py:59-165 ->
  * likelihoods/scalar_continuous.py:139-148).  Xb [B,D], Yc = Yb - m(Xb) [B,P] contiguous,
