@@ -147,9 +147,7 @@ template <typename T>
 int potrf_t(T* A, int64_t n, int64_t rows, int64_t lda, int32_t* info, T* dinv, void* tcws, size_t tcws_bytes,
             cudaStream_t st, bool need_dinv = true, double cond_hint = 0.0);
 
-// tcgen05 (int8-sliced fp64) symmetric rank-k update, gemm_tc.cu
-bool tc_enabled();
-int tc_slices();
+// workspace of the tcgen05 (int8-sliced fp64) trailing updates and of the fp64 detour of fp32 factorisations, potrf.cu
 size_t potrf_tc_ws_bytes(int64_t n, int64_t rows, int dtype);
 
 // tcgen05 kind::tf32 (3xTF32) fp32 GEMM, gemm_tf32.cu

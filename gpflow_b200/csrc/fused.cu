@@ -394,8 +394,7 @@ int svgp_elbo(const gpk_knode* nodes, int n_nodes, const int32_t* dims, const do
   // fvar_p = fvar0 + sum_m (q_sqrt_p^T A)^2   (util.py:149-164) — LTA is never materialised
   // fp32, dense q_sqrt: ALL latents in one batched tcgen05 launch (A split into TF32 planes once, one persistent grid
   // over P x tiles instead of P launches with a 2-wave tail each)
-  static const bool batch_on = []() { const char* e = getenv("GPK_SVGP_BATCHED"); return !(e && e[0] == '0'); }();
-  const bool batched = batch_on && !q_diag && dtype == GPK_F32 && Pl > 1 && M % 256 == 0 &&
+  const bool batched = !q_diag && dtype == GPK_F32 && Pl > 1 && M % 256 == 0 &&
                        gemm_tf32_eligible(M, B, M, nullptr, nullptr, nullptr, 0);
   for (int64_t p = p_begin; p < p_end; ++p) {
     char* fv = (char*)w.fvar + (size_t)(p - p_begin) * B * ts;

@@ -202,7 +202,7 @@ gemm_dmma_kernel(int64_t m, int64_t n, int64_t k, double alpha, const double* A,
 }
 
 // ------------------------------------------------------------------------------------------------
-// generic CUDA-core kernel (fp32 default; fp64 when GPK_FP64_SIMT=1): 128x128x8, 256 threads, 8x8
+// generic CUDA-core kernel (fp32; fp64 runs on the DMMA kernel above): 128x128x8, 256 threads, 8x8
 // ------------------------------------------------------------------------------------------------
 constexpr int SK = 8;
 
@@ -455,12 +455,6 @@ static int launch_skinny(int ta, int64_t m, int n, int64_t k, T alpha, const T* 
 // ------------------------------------------------------------------------------------------------
 // dispatch
 // ------------------------------------------------------------------------------------------------
-static bool fp64_simt() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPK_FP64_SIMT"); v = (e && e[0] == '1') ? 1 : 0; }
-  return v == 1;
-}
-
 template <typename T, int BM, int BN>
 static int launch_simt_shape(int ta, int tb, int64_t m, int64_t n, int64_t k, T alpha, const T* A, int64_t lda,
                              const T* B, int64_t ldb, T beta, T* C, int64_t ldc, int flags, cudaStream_t st, int* hf) {
@@ -561,10 +555,10 @@ int gemm_t(int transa, int transb, int64_t m, int64_t n, int64_t k, T alpha, con
                      (float*)C, ldc, flags, st);
   // work = MACs the launch computes (tiles strictly above the diagonal are skipped for LOWER_ONLY: about half)
   ProfScope ps(PROF_GEMM, st, (double)m * (double)n * (double)k * ((flags & GPK_GEMM_LOWER_ONLY) && m == n ? 0.5 : 1.0));
-  if (sizeof(T) == 8 && !fp64_simt())
-    return launch_dmma(transa, transb, m, n, k, (double)alpha, (const double*)A, lda, (const double*)B, ldb,
-                       (double)beta, (double*)C, ldc, flags, st, hf);
-  return launch_simt<T>(transa, transb, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, flags, st, hf);
+  if constexpr (sizeof(T) == 8)
+    return launch_dmma(transa, transb, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, flags, st, hf);
+  else
+    return launch_simt<T>(transa, transb, m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, flags, st, hf);
 }
 
 template int gemm_t<float>(int, int, int64_t, int64_t, int64_t, float, const float*, int64_t, const float*, int64_t,

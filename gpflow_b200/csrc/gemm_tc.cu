@@ -37,6 +37,9 @@ constexpr int TC_EPI_BYTES = 128 * TC_EPI_ROW;
 constexpr int TC_SMEM_BUDGET = 226 * 1024 - TC_EPI_BYTES;  // pipeline stages: as many as fit (S planes of A and B per stage, tightly packed)
 __host__ __device__ constexpr int tc_stages(int S) { return TC_SMEM_BUDGET / (S * (TC_ATILE + TC_BTILE)) > 6 ? 6 : TC_SMEM_BUDGET / (S * (TC_ATILE + TC_BTILE)); }
 constexpr int TC_TMEM_COLS = 512;
+// CTAs per cluster: the two CTAs of a cluster compute horizontally adjacent tiles and share their A tile by multicast
+// (the kernel is L2 -> SM bandwidth bound)
+constexpr int TC_CL = 2;
 
 // ------------------------------------------------------------------------------------------------
 // scales and slicing
@@ -57,7 +60,7 @@ __global__ void row_exp_kernel(const double* __restrict__ A, int64_t lda, int64_
 }
 
 // dynamic slicing, one CTA per row: rows [row0, row0 + nrows) of the k-range [k0, k0 + K) get the scale of their
-// running maximum over that range (the extra rows below the square part; every row when GPK_TC_STATIC=0)
+// running maximum over that range (the extra rows below the square part)
 __global__ void __launch_bounds__(256)
 slice_rows_kernel(const double* __restrict__ P, int64_t ld, int64_t row0, int64_t nrows, int64_t k0, int64_t K,
                   TcPlanes pl) {
@@ -79,14 +82,15 @@ __host__ __device__ constexpr uint32_t tc_idesc_n(int n) {
 constexpr uint32_t TC_IDESC = tc_idesc_n(TC_BN);
 
 struct TcTileIter {  // identical enumeration in every warp role
-  // Work unit = CL horizontally adjacent tiles (tm, tnb .. tnb+CL-1), one per CTA of a cluster, so the
+  // Work unit = TC_CL horizontally adjacent tiles (tm, tnb .. tnb+TC_CL-1), one per CTA of a cluster, so the
   // cluster shares the A tile (multicast).  Order: pass 0 = the "head" units (first 128 columns) of every
   // row tile, pass 1 = the rest: the next diagonal block's inputs are complete early (look-ahead).
+  static constexpr int64_t head_w = 128 / TC_BN;  // column tiles of the head
   int64_t ntm, ntn;
-  int lower, pass, cl, rank;
+  int lower, pass, rank;
   int64_t tm, tnb, tn, idx;
-  __device__ TcTileIter(int64_t m, int64_t n, int lower_, int cl_, int rank_)
-      : lower(lower_), pass(0), cl(cl_), rank(rank_), tm(0), tnb(-cl_), tn(0), idx(-1) {
+  __device__ TcTileIter(int64_t m, int64_t n, int lower_, int rank_)
+      : lower(lower_), pass(0), rank(rank_), tm(0), tnb(-TC_CL), tn(0), idx(-1) {
     ntm = (m + TC_BM - 1) / TC_BM;
     ntn = (n + TC_BN - 1) / TC_BN;
   }
@@ -100,19 +104,18 @@ struct TcTileIter {  // identical enumeration in every warp role
   __device__ int64_t tn_load() const { return tn < ntn ? tn : ntn - 1; }
   // false for the padding tiles of a unit that sticks out of the (lower-triangular) tile set: computed, not stored
   __device__ bool valid() const { return tn < ncols(tm); }
-  __device__ int64_t head_w() const { return cl > 2 ? cl : 2; }
   // advances to this cluster's next unit; false when exhausted
   __device__ bool next() {
-    const int64_t nunits_grid = gridDim.x / cl, my = blockIdx.x / cl;
+    const int64_t nunits_grid = gridDim.x / TC_CL, my = blockIdx.x / TC_CL;
     for (;;) {
-      tnb += cl;
+      tnb += TC_CL;
       for (;;) {
         if (pass == 0) {
-          const int64_t lim = ncols(tm) < head_w() ? ncols(tm) : head_w();
+          const int64_t lim = ncols(tm) < head_w ? ncols(tm) : head_w;
           if (tm < ntm && tnb >= lim) { ++tm; tnb = 0; continue; }
-          if (tm >= ntm) { pass = 1; tm = 0; tnb = head_w(); continue; }
+          if (tm >= ntm) { pass = 1; tm = 0; tnb = head_w; continue; }
         } else {
-          if (tm < ntm && tnb >= ncols(tm)) { ++tm; tnb = head_w(); continue; }
+          if (tm < ntm && tnb >= ncols(tm)) { ++tm; tnb = head_w; continue; }
           if (tm >= ntm) return false;
         }
         break;
@@ -123,7 +126,7 @@ struct TcTileIter {  // identical enumeration in every warp role
   }
 };
 
-template <int S, bool TS, int CL, bool CAT>
+template <int S>
 __global__ void __launch_bounds__(192, 1)
 syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, int64_t ldc, int64_t m, int64_t n, int KB,
                int lower, int* head_flag) {
@@ -131,12 +134,12 @@ syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, in
   // [32 kb0, 32 (kb0 + KB)) on the diagonal); operands come from the digit-plane store (planes.cuh)
   const double* __restrict__ rowscale = pl.rowscale + rb0 * TC_BM;
   int* err = pl.err;
-  // even S (6): one more accumulator for the (S/2, S/2) digit product (planes.cuh); S = 8 has no TMEM columns left for it
+  // even S (6): one more accumulator for the (S/2, S/2) digit product (planes.cuh)
   constexpr bool SQ = (S == 6);
   constexpr int H = S / 2, NACC = S + (SQ ? 1 : 0);
   extern __shared__ __align__(1024) uint8_t tc_smem[];
   constexpr uint32_t stage_bytes = (uint32_t)S * (TC_ATILE + TC_BTILE);
-  constexpr int TC_STAGES = tc_stages(S);   // S = 7: 5 stages of 42 KB, S = 8: 4 of 48 KB, S = 6: 6 of 36 KB
+  constexpr int TC_STAGES = tc_stages(S);   // S = 7: 5 stages of 42 KB, S = 6: 6 of 36 KB
   constexpr uint32_t stage_stride = (uint32_t)S * (TC_ATILE + TC_BTILE);
   uint8_t* epi_area = tc_smem + TC_STAGES * (size_t)stage_stride;  // [128][TC_EPI_ROW]
   uint8_t* bar_area = epi_area + TC_EPI_BYTES;
@@ -151,7 +154,7 @@ syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, in
     if (blockIdx.x == 0) trace_mark(4, 0);
     for (int i = 0; i < TC_STAGES; ++i) {
       mbar_init(full0 + 8 * i, 1);
-      mbar_init(empty0 + 8 * i, CL);  // every CTA of the cluster releases a stage (A is multicast into all)
+      mbar_init(empty0 + 8 * i, TC_CL);  // every CTA of the cluster releases a stage (A is multicast into all)
     }
     mbar_init(tfull, 1);
     mbar_init(tempty, 128);
@@ -165,19 +168,16 @@ syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, in
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();  // peer barriers initialised before any multicast copy / commit targets them
+  cluster_sync_all();  // peer barriers initialised before any multicast copy / commit targets them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // (programmatic dependent launch: everything above overlapped the tail of the preceding kernel; its results -- the digit
-  // planes of the panel kernel -- may be read from here on.  A no-op when the launch carried no such dependency.)
-  asm volatile("griddepcontrol.wait;" ::: "memory");
   if (threadIdx.x == 0 && blockIdx.x == 0) trace_mark(4, 10);  // prologue done (barriers, TMEM, cluster sync)
-  const int rank = CL > 1 ? (int)cluster_ctarank() : 0;
-  constexpr uint16_t cl_mask = (uint16_t)((1u << CL) - 1);
+  const int rank = (int)cluster_ctarank();
+  constexpr uint16_t cl_mask = (uint16_t)((1u << TC_CL) - 1);
 
   if (__all_sync(0xffffffffu, warp == 0)) {  // vote: the role branch is warp-uniform and the compiler knows it
     // ===== producer (whole warp runs the loop; one elected lane issues the copies) =====
-    TcTileIter it(m, n, lower, CL, rank);
+    TcTileIter it(m, n, lower, rank);
     uint32_t st = 0, ph = 0;
     while (it.next()) {
       const int8_t* a_src = pl.tile(rb0 + it.tm, kb0);
@@ -190,16 +190,12 @@ syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, in
           mbar_expect_tx(fb, stage_bytes);
           const uint32_t sa = smem_u32(tc_smem + (size_t)st * stage_stride);
           const uint32_t sb = sa + S * TC_ATILE;
-          if (CL == 1) {
-            bulk_g2s(sa, a_src + (size_t)kb * S * TC_ATILE, (uint32_t)S * TC_ATILE, fb);
-          } else {
-            // each CTA fetches 1/CL of every A plane (64 of the 128 rows) and multicasts it to the cluster
-            constexpr uint32_t part = TC_ATILE / CL;
+          // each CTA fetches 1/TC_CL of every A plane (64 of the 128 rows) and multicasts it to the cluster
+          constexpr uint32_t part = TC_ATILE / TC_CL;
 #pragma unroll
-            for (int s2 = 0; s2 < S; ++s2)
-              bulk_g2s_mc(sa + s2 * TC_ATILE + rank * part, a_src + ((size_t)kb * S + s2) * TC_ATILE + rank * part, part, fb,
-                          cl_mask);
-          }
+          for (int s2 = 0; s2 < S; ++s2)
+            bulk_g2s_mc(sa + s2 * TC_ATILE + rank * part, a_src + ((size_t)kb * S + s2) * TC_ATILE + rank * part, part, fb,
+                        cl_mask);
 #pragma unroll
           for (int t = 0; t < S; ++t)
             bulk_g2s(sb + t * TC_BTILE, b_src + ((size_t)kb * S + t) * TC_ATILE, TC_BTILE, fb);
@@ -210,7 +206,7 @@ syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, in
     }
   } else if (__all_sync(0xffffffffu, warp == 1)) {
     // ===== MMA issuer (uniform control flow, one elected lane issues) =====
-    TcTileIter it(m, n, lower, CL, rank);
+    TcTileIter it(m, n, lower, rank);
     uint32_t st = 0, ph = 0, tph = 0;
     const uint64_t desc_hi = ((uint64_t)(128 >> 4) << 16) | ((uint64_t)(256 >> 4) << 32) | (1ull << 46);
     while (it.next()) {
@@ -223,69 +219,25 @@ syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, in
         const uint64_t ad0 = desc_hi | (uint64_t)((sa & 0x3FFFFu) >> 4);
         const uint64_t bd0 = ad0 + ((S * TC_ATILE) >> 4);
         if (elect_one()) {
-          if (TS) {
-            // A digit planes -> TMEM (columns S*64 .. S*64 + 8S): every A plane is then read from shared
-            // memory once per k-step instead of once per MMA (S-s times); tcgen05.cp and tcgen05.mma execute
-            // in issue order, so the copy for this k-step queues behind the previous step's MMAs.
-            const uint32_t a_tm = tmem_base + (uint32_t)NACC * TC_BN;
+          // the S-s digit products of A plane s share the A operand and write ADJACENT accumulators, and the B planes are
+          // contiguous in shared memory with the same 8-row-group stride: one MMA with N = 64 (S-s) (split at 256) replaces
+          // S-s MMAs with N = 64 -- 10 instructions per k-step instead of 28 for S = 7
 #pragma unroll
-            for (int s = 0; s < S; ++s) tc_cp_128x256b(a_tm + s * 8, ad0 + (uint64_t)(s * (TC_ATILE >> 4)));
-            if (CAT) {
-              // the S-s digit products of A plane s share the A operand and write ADJACENT accumulators, and the B planes
-              // are contiguous in shared memory with the same 8-row-group stride: one MMA with N = 64 (S-s) (split at
-              // 256) replaces S-s MMAs with N = 64 -- 10 instructions per k-step instead of 28 for S = 7
+          for (int s = 0; s < S; ++s)
 #pragma unroll
-              for (int s = 0; s < S; ++s)
-#pragma unroll
-                for (int t = 0; t + s < S; t += 4) {
-                  int c = (S - s - t) < 4 ? (S - s - t) : 4;
-                  // the square term rides on the MMA of A plane H (B planes 0 .. H instead of 0 .. H-1) except in the first
-                  // k-step, where its accumulator starts from zero while the others of that MMA already hold products
-                  if (SQ && s == H && t == 0 && kb > 0) c = H + 1;
-                  tc_mma_i8_ts(tmem_base + (uint32_t)(s + t) * TC_BN, a_tm + s * 8, bd0 + (uint64_t)(t * (TC_BTILE >> 4)),
-                               tc_idesc_n(TC_BN * c), (kb > 0 || s > 0) ? 1u : 0u);
-                }
-              if (SQ && kb == 0)
-                tc_mma_i8_ts(tmem_base + (uint32_t)S * TC_BN, a_tm + H * 8, bd0 + (uint64_t)(H * (TC_BTILE >> 4)), TC_IDESC, 0u);
-            } else {
-#pragma unroll
-              for (int s = 0; s < S; ++s)
-#pragma unroll
-                for (int t = 0; t + s < S; ++t)
-                  tc_mma_i8_ts(tmem_base + (uint32_t)(s + t) * TC_BN, a_tm + s * 8, bd0 + (uint64_t)(t * (TC_BTILE >> 4)),
-                               TC_IDESC, (kb > 0 || s > 0) ? 1u : 0u);
-              if (SQ)
-                tc_mma_i8_ts(tmem_base + (uint32_t)S * TC_BN, a_tm + H * 8, bd0 + (uint64_t)(H * (TC_BTILE >> 4)), TC_IDESC,
-                             kb > 0 ? 1u : 0u);
+            for (int t = 0; t + s < S; t += 4) {
+              int c = (S - s - t) < 4 ? (S - s - t) : 4;
+              // the square term rides on the MMA of A plane H (B planes 0 .. H instead of 0 .. H-1) except in the first
+              // k-step, where its accumulator starts from zero while the others of that MMA already hold products
+              if (SQ && s == H && t == 0 && kb > 0) c = H + 1;
+              tc_mma_i8(tmem_base + (uint32_t)(s + t) * TC_BN, ad0 + (uint64_t)(s * (TC_ATILE >> 4)),
+                        bd0 + (uint64_t)(t * (TC_BTILE >> 4)), tc_idesc_n(TC_BN * c), (kb > 0 || s > 0) ? 1u : 0u);
             }
-          } else {
-            if (CAT) {
-#pragma unroll
-              for (int s = 0; s < S; ++s)
-#pragma unroll
-                for (int t = 0; t + s < S; t += 4) {
-                  int c = (S - s - t) < 4 ? (S - s - t) : 4;
-                  if (SQ && s == H && t == 0 && kb > 0) c = H + 1;  // + the square term (see the TS branch)
-                  tc_mma_i8(tmem_base + (uint32_t)(s + t) * TC_BN, ad0 + (uint64_t)(s * (TC_ATILE >> 4)),
-                            bd0 + (uint64_t)(t * (TC_BTILE >> 4)), tc_idesc_n(TC_BN * c), (kb > 0 || s > 0) ? 1u : 0u);
-                }
-              if (SQ && kb == 0)
-                tc_mma_i8(tmem_base + (uint32_t)S * TC_BN, ad0 + (uint64_t)(H * (TC_ATILE >> 4)),
-                          bd0 + (uint64_t)(H * (TC_BTILE >> 4)), TC_IDESC, 0u);
-            } else {
-#pragma unroll
-              for (int s = 0; s < S; ++s)
-#pragma unroll
-                for (int t = 0; t + s < S; ++t)
-                  tc_mma_i8(tmem_base + (uint32_t)(s + t) * TC_BN, ad0 + (uint64_t)(s * (TC_ATILE >> 4)),
-                            bd0 + (uint64_t)(t * (TC_BTILE >> 4)), TC_IDESC, (kb > 0 || s > 0) ? 1u : 0u);
-              if (SQ)
-                tc_mma_i8(tmem_base + (uint32_t)S * TC_BN, ad0 + (uint64_t)(H * (TC_ATILE >> 4)),
-                          bd0 + (uint64_t)(H * (TC_BTILE >> 4)), TC_IDESC, kb > 0 ? 1u : 0u);
-            }
-          }
+          if (SQ && kb == 0)
+            tc_mma_i8(tmem_base + (uint32_t)S * TC_BN, ad0 + (uint64_t)(H * (TC_ATILE >> 4)),
+                      bd0 + (uint64_t)(H * (TC_BTILE >> 4)), TC_IDESC, 0u);
           // frees the stage (in every CTA of the cluster) once these copies / MMAs have read it
-          if (CL == 1) tc_commit(empty0 + 8 * st); else tc_commit_mc(empty0 + 8 * st, cl_mask);
+          tc_commit_mc(empty0 + 8 * st, cl_mask);
         }
         __syncwarp();
         if (++st == TC_STAGES) { st = 0; ph ^= 1; }
@@ -305,7 +257,7 @@ syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, in
     // (The previous read-modify-write epilogue -- 16-byte loads / stores of a thread's own row, 32 lines per warp
     // instruction -- took 7.7 us per tile on the LSU: profiles/r2/trace_c2_phases.csv.)
     const int q = warp & 3;  // TMEM lane quarter this warp may access
-    TcTileIter it(m, n, lower, CL, rank);
+    TcTileIter it(m, n, lower, rank);
     uint32_t tph = 0;
     const bool vec_ok = ((ldc & 1) == 0) && ((reinterpret_cast<uintptr_t>(C) & 15) == 0);
     double* srow = reinterpret_cast<double*>(epi_area + (size_t)(q * 32 + lane) * TC_EPI_ROW);
@@ -395,7 +347,7 @@ syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, in
   tc_fence_before();
   __syncthreads();
   if (threadIdx.x == 0 && (blockIdx.x == 0 || blockIdx.x == gridDim.x - 1)) trace_mark(4, blockIdx.x == 0 ? 2 : 3);
-  if (CL > 1) cluster_sync_all();  // no CTA leaves while a peer may still multicast into its shared memory
+  cluster_sync_all();  // no CTA leaves while a peer may still multicast into its shared memory
   if (warp == 1) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TC_TMEM_COLS)
                  : "memory");
@@ -405,64 +357,25 @@ syrk_i8_kernel(TcPlanes pl, int64_t rb0, int64_t kb0, double* __restrict__ C, in
 // ------------------------------------------------------------------------------------------------
 // host
 // ------------------------------------------------------------------------------------------------
-// GPK_TC_SLICES pins the number of digit planes (6..8); 0 = chosen per factorisation (potrf.cu::pick_slices)
-int tc_slices() {
-  static int s = -1;
-  if (s < 0) {
-    const char* e = getenv("GPK_TC_SLICES");
-    s = e ? atoi(e) : 0;
-    if (s != 0 && s < 6) s = 6;
-    if (s > TC_MAXS) s = TC_MAXS;
-  }
-  return s;
-}
-
 int trace_set_tc(TraceBuf tb) {
   GPK_CUDA_OK(cudaMemcpyToSymbol(g_trace, &tb, sizeof(tb)));
   return 0;
 }
 
-bool tc_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("GPK_FP64_ENGINE");
-    v = (e && (strcmp(e, "dmma") == 0 || strcmp(e, "simt") == 0)) ? 0 : 1;
-  }
-  return v == 1;
-}
-
-static bool tc_static_scales() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPK_TC_STATIC"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
-}
-
-static bool tc_rect() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPK_TC_RECT"); v = (e && e[0] == '1') ? 1 : 0; }
-  return v == 1;
-}
-
-static size_t tc_tiles_total(int64_t rbt, int64_t nbk) {
-  return (size_t)(tc_rect() ? rbt * 4 * nbk : plane_prefix(rbt, nbk));
-}
-
 size_t tc_planes_bytes(int64_t n, int64_t rows) {
   const int64_t nbk = (n + TC_BM - 1) / TC_BM, rbt = (rows + TC_BM - 1) / TC_BM;
-  return align_up(tc_tiles_total(rbt, nbk) * TC_MAXS * TC_ATILE, 256) + align_up((size_t)rbt * TC_BM * sizeof(double), 256) + 256;
+  return align_up((size_t)plane_prefix(rbt, nbk) * TC_MAXS * TC_ATILE, 256) + align_up((size_t)rbt * TC_BM * sizeof(double), 256) + 256;
 }
 
 TcPlanes tc_planes_layout(void* ws, int64_t n, int64_t rows, int S) {
   const int64_t nbk = (n + TC_BM - 1) / TC_BM, rbt = (rows + TC_BM - 1) / TC_BM;
   TcPlanes pl;
   pl.planes = (int8_t*)ws;
-  pl.rowscale = (double*)((char*)ws + align_up(tc_tiles_total(rbt, nbk) * TC_MAXS * TC_ATILE, 256));
-  pl.rect = tc_rect();
+  pl.rowscale = (double*)((char*)ws + align_up((size_t)plane_prefix(rbt, nbk) * TC_MAXS * TC_ATILE, 256));
   pl.err = (int*)((char*)pl.rowscale + align_up((size_t)rbt * TC_BM * sizeof(double), 256));
   pl.S = S;
   pl.nbk = nbk;
   pl.n_sq = n;
-  pl.is_static = tc_static_scales();
   return pl;
 }
 
@@ -504,65 +417,40 @@ int syrk_tc_planes(double* C, int64_t ldc, int64_t m, int64_t n, const TcPlanes&
   // Both operands from shared memory with the digit products of one A plane CONCATENATED along N (one MMA of N up to 256
   // instead of up to four of N = 64): scripts/mb_mma.cu measures 52.9 cycles per N = 64 SS MMA against a floor of 32,
   // but 128.0 per N = 256 MMA (= the floor), and the tcgen05.cp of the TS form costs 137 cycles per k-step on top.
-  // C2: 8.70 ms (TS, N = 64) -> 8.14 ms (SS, concatenated).  GPK_TC_A_TMEM=1 / GPK_TC_CAT=0 select the older forms.
-  // Clusters of 2 CTAs multicast the shared A tile (the kernel is L2->SM bandwidth bound); GPK_TC_CLUSTER=1 disables.
-  static const bool ts = []() { const char* e = getenv("GPK_TC_A_TMEM"); return e && e[0] == '1'; }();
-  static const int cl = []() {
-    const char* e = getenv("GPK_TC_CLUSTER");
-    return (e && e[0] == '1') ? 1 : (e && e[0] == '4') ? 4 : 2;
-  }();
-  // number of work units (CL adjacent tiles)
+  // C2: 8.70 ms (TS, N = 64) -> 8.14 ms (SS, concatenated).
+  // number of work units (TC_CL adjacent tiles)
   const int64_t ntm = (m + TC_BM - 1) / TC_BM, ntn = (n + TC_BN - 1) / TC_BN;
   int64_t nunits = 0;
   for (int64_t t = 0; t < ntm; ++t) {
     const int64_t nc = lower ? (2 * t + 2 < ntn ? 2 * t + 2 : ntn) : ntn;
-    nunits += (nc + cl - 1) / cl;
+    nunits += (nc + TC_CL - 1) / TC_CL;
   }
   int grid = tc_num_sms() - (hf ? 1 : 0);  // look-ahead: leave one SM for the concurrent leaf kernel
-  grid = grid / cl * cl;
-  if (nunits * cl < grid) grid = (int)(nunits * cl);
+  grid = grid / TC_CL * TC_CL;
+  if (nunits * TC_CL < grid) grid = (int)(nunits * TC_CL);
   if (grid < 1) return 0;
   const int KBn = (int)(K / TC_KB);
   // issued int8 MACs: every tile of every unit (padding tiles included) x k-steps x S(S+1)/2 digit products
-  ProfScope ps(PROF_TC, st, (double)nunits * cl * KBn * (S * (S + 1) / 2 + (S == 6 ? 1 : 0)) * (double)(TC_BM * TC_BN * TC_KB));
-  static const bool pdl = []() { const char* e = getenv("GPK_TC_PDL"); return e && e[0] == '1'; }();  // off: see potrf_panel_kernel
+  ProfScope ps(PROF_TC, st, (double)nunits * TC_CL * KBn * (S * (S + 1) / 2 + (S == 6 ? 1 : 0)) * (double)(TC_BM * TC_BN * TC_KB));
   auto launch = [&](auto kern) -> int {
-    static_cast<void>(0);
     GPK_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3(192);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
-    cudaLaunchAttribute at[2];
+    cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = (unsigned)cl;
+    at[0].val.clusterDim.x = (unsigned)TC_CL;
     at[0].val.clusterDim.y = 1;
     at[0].val.clusterDim.z = 1;
-    at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
-    cfg.numAttrs = pdl ? 2 : 1;
+    cfg.numAttrs = 1;
     GPK_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, pl, rb0, kb0, C, ldc, m, n, KBn, lower, hf));
     count_launch();
     return 0;
   };
-  static const bool cat = []() { const char* e = getenv("GPK_TC_CAT"); return !(e && e[0] == '0'); }();
-#define GPK_TC_PICK(SS, TT, CC) (cat ? launch(syrk_i8_kernel<SS, TT, CC, true>) : launch(syrk_i8_kernel<SS, TT, CC, false>))
-  if (cl == 4) {
-    if (S == 6) return ts ? GPK_TC_PICK(6, true, 4) : GPK_TC_PICK(6, false, 4);
-    if (S == 7) return ts ? GPK_TC_PICK(7, true, 4) : GPK_TC_PICK(7, false, 4);
-    return GPK_TC_PICK(8, false, 4);
-  }
-  if (cl == 2) {
-    if (S == 6) return ts ? GPK_TC_PICK(6, true, 2) : GPK_TC_PICK(6, false, 2);
-    if (S == 7) return ts ? GPK_TC_PICK(7, true, 2) : GPK_TC_PICK(7, false, 2);
-    return GPK_TC_PICK(8, false, 2);
-  }
-  if (S == 6) return ts ? GPK_TC_PICK(6, true, 1) : GPK_TC_PICK(6, false, 1);
-  if (S == 7) return ts ? GPK_TC_PICK(7, true, 1) : GPK_TC_PICK(7, false, 1);
-  return GPK_TC_PICK(8, false, 1);
-#undef GPK_TC_PICK
+  return S == 6 ? launch(syrk_i8_kernel<6>) : launch(syrk_i8_kernel<7>);
 }
 
 }  // namespace gpk

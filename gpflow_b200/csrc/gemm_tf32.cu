@@ -422,12 +422,6 @@ int tf32_reserve(size_t bytes, cudaStream_t st) {
   return rc;
 }
 
-bool tf32_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPK_FP32_ENGINE"); v = (e && strcmp(e, "simt") == 0) ? 0 : 1; }
-  return v == 1;
-}
-
 static int tf_num_sms() {
   static int n = 0;
   if (n == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev); if (n <= 0) n = 148; }
@@ -437,7 +431,6 @@ static int tf_num_sms() {
 // eligibility: big enough to amortise the pre-pass; no aliasing of C with an operand (the pre-pass makes
 // copies, but in-place callers rely on tile-local ordering which the persistent kernel does not give)
 bool gemm_tf32_eligible(int64_t m, int64_t n, int64_t k, const void* A, const void* B, const void* C, int flags) {
-  if (!tf32_enabled()) return false;
   if (k < 64 || m < 64 || n < 64) return false;
   if ((double)m * n * k < 2.0e8) return false;
   (void)A; (void)B; (void)C; (void)flags;
@@ -476,9 +469,8 @@ int gemm_tf32(int transa, int transb, int64_t m, int64_t n, int64_t k, float alp
   }
   const int lower = (flags & GPK_GEMM_LOWER_ONLY) ? 1 : 0;
   const int64_t ntm = mpad / TF_BM, ntn = npad / TF_BN;
-  // clusters of 2 row tiles share the B planes by multicast (GPK_TF32_CLUSTER=1 disables); a single row tile has no pair
-  static const int cl_env = []() { const char* e = getenv("GPK_TF32_CLUSTER"); return (e && e[0] == '1') ? 1 : 2; }();
-  const int cl = ntm >= 2 ? cl_env : 1;
+  // clusters of 2 row tiles share the B planes by multicast; a single row tile has no pair
+  const int cl = ntm >= 2 ? 2 : 1;
   int64_t nunits = 0;  // work units of cl vertically adjacent row tiles (the lowest tile decides whether a unit is needed)
   for (int64_t tn = 0; tn < ntn; ++tn)
     for (int64_t t0 = 0; t0 < ntm; t0 += cl)

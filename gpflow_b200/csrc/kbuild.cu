@@ -788,8 +788,8 @@ static int kbuild_fast_launch(const KProg& p, const void* X, int64_t N, int64_t 
   ProfScope ps(PROF_KBUILD, st);
   const int vec_ok = ((uintptr_t)K % 16 == 0) && ((ldk * sizeof(T)) % 16 == 0);
   const int mode = p.symmetric ? (lower ? 1 : 2) : 0;
-  // resident CTAs per SM the kernel is compiled for: 2 (<= 128 registers) or 3 (<= 80); GPK_KF_MINB overrides
-  static const bool minb2 = []() { const char* e = getenv("GPK_KF_MINB"); return e ? e[0] == '2' : sizeof(T) == 8; }();
+  // resident CTAs per SM the kernel is compiled for: 2 (<= 128 registers) for fp64, 3 (<= 80) for fp32
+  constexpr int minb = sizeof(T) == 8 ? 2 : 3;
   // fold c / lengthscale^2 into the per-dimension weights (applied to both operands): x = c r2 comes out of
   // the norm expansion with no further scaling
 #define GPK_KF(TY)                                                                                         \
@@ -798,9 +798,7 @@ static int kbuild_fast_launch(const KProg& p, const void* X, int64_t N, int64_t 
     const double f = sqrt(q.l_scale[0] * kf_fold<TY>());                                                   \
     for (int d = 0; d < q.g_ndims[0]; ++d) q.w[d] *= f;                                                    \
     q.l_scale[0] = 1.0;                                                                                    \
-    if (minb2)                                                                                             \
-      return kbuild_fast_go<T, TY, 2>(q, X, N, ldx, X2, N2, ldx2, K, ldk, mode, diag_scalar, diag_vec, vec_ok, st); \
-    return kbuild_fast_go<T, TY, 3>(q, X, N, ldx, X2, N2, ldx2, K, ldk, mode, diag_scalar, diag_vec, vec_ok, st); \
+    return kbuild_fast_go<T, TY, minb>(q, X, N, ldx, X2, N2, ldx2, K, ldk, mode, diag_scalar, diag_vec, vec_ok, st); \
   } while (0)
   switch (p.l_type[0]) {
     case GPK_K_RBF: GPK_KF(GPK_K_RBF);
@@ -848,8 +846,7 @@ int kbuild_impl(const gpk_knode* nodes, int n_nodes, const int32_t* dims, const 
   KProg p;
   GPK_TRY(compile_kprog(nodes, n_nodes, dims, ard, D, p));
   p.symmetric = sym ? 1 : 0;
-  static const bool no_fast = getenv("GPK_KBUILD_GENERIC") != nullptr;
-  if (fast_path_ok(p) && !no_fast) {
+  if (fast_path_ok(p)) {
     if (dtype == GPK_F64)
       return kbuild_fast_launch<double>(p, X, N, ldx, X2, N2, ldx2, K, ldk, uplo == GPK_LOWER, diag_scalar, diag_vec, st);
     return kbuild_fast_launch<float>(p, X, N, ldx, X2, N2, ldx2, K, ldk, uplo == GPK_LOWER, diag_scalar, diag_vec, st);

@@ -26,7 +26,7 @@ namespace gpk {
 constexpr int TC_BM = 128, TC_BN = 64, TC_KB = 32;   // CTA tile of the update, bytes (= int8 elements) per k-step
 constexpr int TC_ATILE = TC_BM * TC_KB;              // 4096 B per digit plane of a 128-row tile
 constexpr int TC_BTILE = TC_BN * TC_KB;              // 2048 B (one half of a 128-row tile)
-constexpr int TC_MAXS = 8;
+constexpr int TC_MAXS = 8;                           // planes the store is sized for (S <= 7 is used)
 
 // byte offset of element (row r in [0,128), k in [0,32)) inside one digit-plane tile:
 // canonical no-swizzle K-major UMMA layout ((8,n),2):((1,SBO),LBO) in 16-byte units, LBO = 8, SBO = 16
@@ -107,14 +107,11 @@ struct TcPlanes {
   int8_t* planes = nullptr;   // digit planes, triangular tile packing
   double* rowscale = nullptr; // [rows_pad]: 2^(e_i - 6)
   int* err = nullptr;         // device word: protocol error code of the tcgen05 kernel (bounded waits)
-  int S = 7;
+  int S = 7;                  // digit planes per element: 6 or 7
   int64_t nbk = 0;            // 128-column blocks of the square part
   int64_t n_sq = 0;           // rows >= n_sq are "extra" rows (dynamic scales)
-  bool is_static = true;      // false: every update re-slices its operand rows (GPK_TC_STATIC=0)
-  bool rect = false;          // experiment (GPK_TC_RECT=1): rectangular instead of triangular tile packing
   __device__ __host__ int8_t* tile(int64_t rb, int64_t kb) const {
-    const int64_t pre = rect ? rb * 4 * nbk : plane_prefix(rb, nbk);
-    return planes + (size_t)(pre + kb) * S * TC_ATILE;
+    return planes + (size_t)(plane_prefix(rb, nbk) + kb) * S * TC_ATILE;
   }
 };
 

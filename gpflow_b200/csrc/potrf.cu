@@ -155,32 +155,9 @@ __device__ __forceinline__ int warp_chol32(T* S, int jb, T* ldiag) {
   for (int c = 0; c < 32; ++c) a[c] = c <= lane ? S[(jb + lane) * LS + jb + c] : T(0);
   int bad = 0;
   T my_inv = T(1), my_diag = T(1);
-#ifndef GPK_CHOL32_VARIANT
-#define GPK_CHOL32_VARIANT 1  // measured on B200, cycles per block: variant 1 8.1k, variant 3 8.4k, variant 0 9.4k, variant 2 9.8k
-#endif
-#if GPK_CHOL32_VARIANT == 0
-  // Right-looking, fully unrolled.  Alternatives measured (scripts/chol32_variants.sh): 8-column blocking and
-  // left-looking columns with four split partial sums.
-#pragma unroll
-  for (int k = 0; k < 32; ++k) {
-    T d = __shfl_sync(0xffffffffu, a[k], k);
-    if (!(d > T(0))) {  // non-positive or NaN pivot
-      if (bad == 0) bad = k + 1;
-      d = T(1);
-    }
-    const T inv = rsqrt_t<T>(d);
-    if (lane == k) { my_inv = inv; my_diag = d * inv; }
-    a[k] *= inv;  // l_ik for lane i > k; rows above hold zeros
-#pragma unroll
-    for (int j = 0; j < 32; ++j)
-      if (j > k) {
-        const T ljk = __shfl_sync(0xffffffffu, a[k], j);
-        if (lane >= j) a[j] -= a[k] * ljk;
-      }
-  }
-#elif GPK_CHOL32_VARIANT == 1
   // left-looking: corrections from columns < j-1 go into four independent partial sums, only the last one sits on
-  // the pivot chain; entries above the diagonal accumulate harmless garbage (never read or stored)
+  // the pivot chain; entries above the diagonal accumulate harmless garbage (never read or stored).  Measured on B200,
+  // cycles per block: 8.1k (right-looking: 9.4k, blocked by 8 columns: 9.8k, pivots formed by every lane: 8.4k)
 #pragma unroll
   for (int j = 0; j < 32; ++j) {
     if (j >= 2) {
@@ -206,75 +183,6 @@ __device__ __forceinline__ int warp_chol32(T* S, int jb, T* ldiag) {
     if (lane == j) { my_inv = inv; my_diag = d * inv; }
     a[j] *= inv;
   }
-#elif GPK_CHOL32_VARIANT == 3
-  // variant 1 with ONE shuffle on the pivot chain instead of two: every lane forms the pivot d_j = A_jj - sum_k l_jk^2
-  // itself from the row-j entries it receives for the dot product anyway (same products, same summation order as lane
-  // j's own diagonal entry: bit-identical pivots), A_jj is a broadcast load from the still untouched shared block.
-  // Measured 3 % SLOWER than variant 1: the 496 extra DFMAs cost more issue slots than the shuffle latency they remove.
-#pragma unroll
-  for (int j = 0; j < 32; ++j) {
-    T dd = S[(jb + j) * LS + jb + j];
-    if (j >= 2) {
-      T p0 = T(0), p1 = T(0), p2 = T(0), p3 = T(0), s0 = T(0), s1 = T(0), s2 = T(0), s3 = T(0);
-#pragma unroll
-      for (int k = 0; k < 32; ++k)
-        if (k < j - 1) {
-          const T ljk = __shfl_sync(0xffffffffu, a[k], j);
-          if ((k & 3) == 0) { p0 = fma(a[k], ljk, p0); s0 = fma(ljk, ljk, s0); }
-          else if ((k & 3) == 1) { p1 = fma(a[k], ljk, p1); s1 = fma(ljk, ljk, s1); }
-          else if ((k & 3) == 2) { p2 = fma(a[k], ljk, p2); s2 = fma(ljk, ljk, s2); }
-          else { p3 = fma(a[k], ljk, p3); s3 = fma(ljk, ljk, s3); }
-        }
-      a[j] -= (p0 + p1) + (p2 + p3);
-      dd -= (s0 + s1) + (s2 + s3);
-    }
-    if (j >= 1) {
-      const T l = __shfl_sync(0xffffffffu, a[j - 1], j);
-      a[j] = fma(-a[j - 1], l, a[j]);
-      dd = fma(-l, l, dd);
-    }
-    T d = dd;
-    if (!(d > T(0))) {
-      if (bad == 0) bad = j + 1;
-      d = T(1);
-    }
-    const T inv = rsqrt_t<T>(d);
-    if (lane == j) { my_inv = inv; my_diag = d * inv; }
-    a[j] *= inv;
-  }
-#else
-  // blocked by 8 columns: inside a block each pivot updates only the block's remaining columns; the columns to the
-  // right receive the block's 8 rank-1 updates afterwards (same subtraction order: bit-identical to variant 0)
-#pragma unroll
-  for (int kb = 0; kb < 32; kb += 8) {
-#pragma unroll
-    for (int k = kb; k < kb + 8; ++k) {
-      T d = __shfl_sync(0xffffffffu, a[k], k);
-      if (!(d > T(0))) {
-        if (bad == 0) bad = k + 1;
-        d = T(1);
-      }
-      const T inv = rsqrt_t<T>(d);
-      if (lane == k) { my_inv = inv; my_diag = d * inv; }
-      a[k] *= inv;
-#pragma unroll
-      for (int j = kb; j < kb + 8; ++j)
-        if (j > k) {
-          const T ljk = __shfl_sync(0xffffffffu, a[k], j);
-          if (lane >= j) a[j] -= a[k] * ljk;
-        }
-    }
-#pragma unroll
-    for (int j = 0; j < 32; ++j)
-      if (j >= kb + 8) {
-#pragma unroll
-        for (int k = kb; k < kb + 8; ++k) {
-          const T ljk = __shfl_sync(0xffffffffu, a[k], j);
-          if (lane >= j) a[j] -= a[k] * ljk;
-        }
-      }
-  }
-#endif
 #pragma unroll
   for (int c = 0; c < 32; ++c)
     if (c < lane) S[(jb + lane) * LS + jb + c] = a[c];
@@ -733,10 +641,6 @@ potrf_panel_kernel(double* __restrict__ B, int64_t ldb, int64_t rows, const doub
   const int64_t r0 = critical ? (int64_t)blockIdx.x * PCR : (int64_t)ncrit * PCR + (int64_t)(blockIdx.x - ncrit) * PR;
   const bool wact = w * 8 < nrows_cta;  // warps beyond the CTA's rows only help with the cooperative loads / emission
   const int trace_id = fu.C ? 2 : 3;
-  // programmatic dependent launch (experiment, GPK_TC_PDL=1): the tcgen05 update behind a plain panel is then launched with
-  // the stream-serialisation attribute and blocks in griddepcontrol.wait until this grid has completed.  Measured 1 %
-  // slower per evaluation: the early-resident update CTAs take the free SMs and the next leaf starts late.
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   if (tid == 0 && blockIdx.x == 0) trace_mark(trace_id, 0);
   double* Bw = Bs + (w * 8) * PLB;  // this warp's 8 rows
   // Operands (A^-1, D^-1, C: 3 x 32 KB) and the CTA's rows (up to 64 KB) come in as 16-byte asynchronous copies, all in
@@ -1046,12 +950,8 @@ static int leaf_attr() {
 
 static inline int64_t split_point(int64_t n) { return ((n / NB + 1) / 2) * NB; }
 
-// Updates with K below this use the DMMA kernel (slicing + epilogue overhead of the int8 path); GPK_TC_MIN_K overrides.
-static int64_t tc_min_k() {
-  static int64_t v = 0;
-  if (!v) { const char* e = getenv("GPK_TC_MIN_K"); v = e ? atoll(e) : 256; if (v < 128) v = 128; }
-  return v;
-}
+// Updates with K below this use the DMMA kernel (slicing + epilogue overhead of the int8 path).
+constexpr int64_t TC_MIN_K = 256;
 
 // ---- look-ahead context ------------------------------------------------------------------------------
 // The trailing update U (main stream) and the next diagonal-block factorisation (side stream) overlap:
@@ -1074,12 +974,6 @@ struct LookAhead {
   bool fuse = false;       // slim + look-ahead: the K = 128 updates are applied by the panel kernel itself
   TcPlanes pl;             // digit-plane store of this factorisation (pl.planes == nullptr: tcgen05 updates off)
 };
-
-static bool lookahead_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPK_LOOKAHEAD"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
-}
 
 static int num_sms() {  // of the CURRENT device (a process may drive several)
   int dev = 0, n = 0;
@@ -1119,25 +1013,13 @@ static int flight_mark(cudaStream_t st) {
   return 0;
 }
 
-static bool flaghop_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPK_FLAG_HOPS"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
-}
-
-static bool fuse_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPK_PANEL_FUSE"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
-}
-
 static int lookahead_init(LookAhead& la, int* flag, cudaStream_t st) {
   // one side stream + event set per (device, caller stream): independent factorisations issued on
   // different streams (e.g. one model per output) never share look-ahead state
   struct Res { cudaStream_t side; cudaEvent_t ev[3]; };
   static std::map<std::pair<int, cudaStream_t>, Res> pool;
   static std::mutex mu;
-  if (!lookahead_enabled() || !flag) return 0;
+  if (!flag) return 0;
   int dev = 0;
   GPK_CUDA_OK(cudaGetDevice(&dev));
   std::lock_guard<std::mutex> lock(mu);
@@ -1169,7 +1051,7 @@ int lookahead_warm(cudaStream_t st) {
 // int32 accumulators: 128 * 128 * K * S < 2^31 (radix-256 digits; tests/test_digit_slicing_model.py); deeper updates use DMMA
 template <typename T>
 static bool tc_update_eligible(const LookAhead& la, int64_t m, int64_t n, int64_t K) {
-  return sizeof(T) == 8 && la.pl.planes && K >= tc_min_k() && K % 32 == 0 && n <= m && K * la.pl.S * 16384 < (1ll << 31);
+  return sizeof(T) == 8 && la.pl.planes && K >= TC_MIN_K && K % 32 == 0 && n <= m && K * la.pl.S * 16384 < (1ll << 31);
 }
 
 template <typename T>
@@ -1178,10 +1060,10 @@ static int trailing_update(T* C, int64_t ldc, int64_t m, int64_t n, const T* P, 
   GemmOpts opts;
   const bool use_tc = tc_update_eligible<T>(la, m, n, K);
   if (use_tc) {
-    // operand rows without a static scale: the extra rows below the square part (or every row, GPK_TC_STATIC=0)
+    // operand rows without a static scale: the extra rows below the square part
     const int64_t r0 = col0 + K;
-    const int64_t dyn0 = la.pl.is_static ? (la.pl.n_sq > r0 ? la.pl.n_sq : r0) : r0;
-    if (dyn0 < r0 + m && !(la.pl.is_static && la.dyn_k0 == col0 && la.dyn_K == K))  // (else: the last panel kernel did it)
+    const int64_t dyn0 = la.pl.n_sq > r0 ? la.pl.n_sq : r0;
+    if (dyn0 < r0 + m && !(la.dyn_k0 == col0 && la.dyn_K == K))  // (else: the last panel kernel did it)
       GPK_TRY(tc_slice_rows((const double*)P + (dyn0 - r0) * ldp, ldp, dyn0, r0 + m - dyn0, col0, K, la.pl, st));
   }
   if (la.enabled) {
@@ -1201,13 +1083,7 @@ static int trailing_update(T* C, int64_t ldc, int64_t m, int64_t n, const T* P, 
 }
 
 // (fp32 factorisations by way of the fp64 path: potrf_f32_via_f64 below)
-static bool f32_via_f64_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPK_F32_VIA_F64"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
-}
-
-static bool f32_detour_applies(int64_t n, int64_t rows) { return rows <= n && n >= 512 && n <= 65535 && f32_via_f64_enabled(); }
+static bool f32_detour_applies(int64_t n, int64_t rows) { return rows <= n && n >= 512 && n <= 65535; }
 struct F32Detour { int64_t ld64; size_t a_bytes, d_bytes, p_bytes; };
 static F32Detour f32_detour_layout(int64_t n) {
   F32Detour d;
@@ -1224,7 +1100,7 @@ size_t potrf_tc_ws_bytes(int64_t n, int64_t rows, int dtype) {
     const F32Detour L = f32_detour_layout(n);
     return L.a_bytes + L.d_bytes + L.p_bytes;
   }
-  if (n < 2 * 128) return 0;  // sized for any GPK_TC_MIN_K >= 128
+  if (n < 2 * 128) return 0;  // reserved from n >= 256; the updates use the planes once split_point(n) >= TC_MIN_K (n >= 384)
   return tc_planes_bytes(n, rows);
 }
 
@@ -1277,7 +1153,7 @@ static int potrf_block(T* A, int64_t n, int64_t rows, int64_t lda, int32_t* info
   }
   PanelEmit em{};
   PanelFuse fu{};
-  if (la.slim && la.pl.is_static) {  // (GPK_TC_STATIC=0: every update slices its own operand rows instead)
+  if (la.slim) {
     em.pl = la.pl;
     em.row_g0 = col0 + n;
     em.col_g0 = col0;
@@ -1380,24 +1256,16 @@ static int potrf_rec(T* A, int64_t n, int64_t rows, int64_t lda, int32_t* info, 
   return potrf_rec<T>(A + n1 * lda + n1, n - n1, rows - n1, lda, info, dinv, col0 + n1, la, st, fk0, fK);
 }
 
-static bool slim_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPK_SLIM_LEAF"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
-}
-
 // Number of base-256 digit planes of the tcgen05 trailing updates from what the caller knows about the conditioning
 // (cond = max_i A_ii / lambda_min, e.g. (kernel variance + noise) / noise for GPR).  Measured with the NumPy emulation
 // of this factorisation (scripts/radix_study.py; numerically low-rank matrices, static scales): S = 6 (+ the (3,3) product)
 // moves L by ~1e-12 cond relative and the LML by <= 2e-8 relative up to cond 1e4; S = 7 resolves 2^-54 of the row scale and
 // stays within ~3x of plain fp64 arithmetic for every conditioning tried (1e1 .. 1e8), so it serves everything else,
-// including an unknown conditioning (a bare gpk_potrf).  GPK_TC_SLICES pins S (6 .. 8).
+// including an unknown conditioning (a bare gpk_potrf).
 static int g_last_slices = 0;  // diagnostic: digit planes of the most recent fp64 factorisation (0 = DMMA / none)
 int potrf_last_slices() { return g_last_slices; }
 
 static int pick_slices(double cond_hint) {
-  const int pinned = tc_slices();
-  if (pinned) return pinned;
   return (cond_hint > 0.0 && cond_hint <= 1e4) ? 6 : 7;
 }
 
@@ -1408,7 +1276,7 @@ static int pick_slices(double cond_hint) {
 // rounded back; the fp32 block inverses the triangular solves consume are recomputed from the rounded factor.  (The factor
 // is the correctly rounded fp64 factor instead of an fp32-accumulated one.)  The fp64 copy, its block-inverse slots and its
 // digit planes live in the CALLER's workspace: potrf_tc_ws_bytes(n, rows, GPK_F32) is part of gpk_potrf_ws / the fused
-// objectives' workspace queries.  GPK_F32_VIA_F64=0 keeps the fp32 kernels.
+// objectives' workspace queries.
 __global__ void widen_lower_kernel(const float* __restrict__ A, int64_t lda, double* __restrict__ B, int64_t ldb, int64_t n) {
   const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y;
   if (c <= r && c < n) B[r * ldb + c] = (double)A[r * lda + c];
@@ -1454,18 +1322,18 @@ int potrf_t(T* A, int64_t n, int64_t rows, int64_t lda, int32_t* info, T* dinv, 
   int* flag = reinterpret_cast<int*>(reinterpret_cast<char*>(dinv) + (size_t)((n + NB - 1) / NB) * NB * NB * sizeof(T));
   if (n > NB) GPK_TRY(lookahead_init(la, flag, st));
   if (la.enabled) GPK_CUDA_OK(cudaMemsetAsync(la.flag, 0, 4 * sizeof(int), st));  // counters run up from here (la.base1 / base2)
-  la.slim = sizeof(T) == 8 && n > NB && slim_enabled();
-  la.fuse = la.slim && la.enabled && fuse_enabled();
+  la.slim = sizeof(T) == 8 && n > NB;
+  la.fuse = la.slim && la.enabled;
   std::unique_lock<std::mutex> flight_lock(g_flight_mu, std::defer_lock);
   if (la.enabled) flight_lock.lock();
-  la.flaghop = la.slim && la.enabled && flaghop_enabled() && flight_alone(st);
-  // digit-plane store for the tcgen05 trailing updates: fp64, slim panels (they emit the planes), n >= 2 tc_min_k
+  la.flaghop = la.slim && la.enabled && flight_alone(st);
+  // digit-plane store for the tcgen05 trailing updates: fp64, slim panels (they emit the planes), split_point(n) >= TC_MIN_K
   const int S = pick_slices(cond_hint);
   if (sizeof(T) == 8) g_last_slices = 0;
-  if (S && la.slim && tcws && tc_enabled() && split_point(n) >= tc_min_k() && tcws_bytes >= tc_planes_bytes(n, rows)) {
+  if (la.slim && tcws && split_point(n) >= TC_MIN_K && tcws_bytes >= tc_planes_bytes(n, rows)) {
     la.pl = tc_planes_layout(tcws, n, rows, S);
     g_last_slices = S;
-    if (la.pl.is_static) GPK_TRY(tc_row_exponents((const double*)A, lda, la.pl, st));  // from the ORIGINAL diagonal
+    GPK_TRY(tc_row_exponents((const double*)A, lda, la.pl, st));  // from the ORIGINAL diagonal
   }
   GPK_TRY(potrf_rec<T>(A, n, rows, lda, info, dinv, 0, la, st));
   if (la.flaghop && la.side_started) {  // the caller's stream continues behind the last leaf

@@ -10,6 +10,21 @@ void count_launch() {}
 }  // namespace gpk
 using namespace gpk;
 
+// TS form: A operand read from TMEM (written there by tcgen05.cp), B from shared memory
+__device__ __forceinline__ void tc_mma_i8_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc,
+                                             uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], [%1], %2, %3, {%5, %6, %7, %8}, p;\n\t}"
+      ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(0u), "r"(0u), "r"(0u), "r"(0u)
+      : "memory");
+}
+// shared memory (matrix descriptor) -> TMEM, 128 lanes x 256 bits (32 bytes per row = one K=32 int8 step)
+__device__ __forceinline__ void tc_cp_128x256b(uint32_t d_tmem, uint64_t sdesc) {
+  asm volatile("tcgen05.cp.cta_group::1.128x256b [%0], %1;" ::"r"(d_tmem), "l"(sdesc) : "memory");
+}
+
 __host__ __device__ constexpr uint32_t idesc_n(int n) {
   return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
 }

@@ -395,8 +395,8 @@ def test_c2_full_size_factor_residual(cuda_device):
     num = float(ops.reduce(ops.SUMSQ, R, R.numel())) ** 0.5
     den = float(ops.reduce(ops.SUMSQ, K, K.numel())) ** 0.5
     # digit planes with STATIC row scales 2^ceil(log2 sqrt(K_ii)) (csrc/planes.cuh): rows of L are usually well below
-    # sqrt(K_ii), so a few leading digit bits are unused -- measured 6e-13 here (4e-14 with per-update row maxima,
-    # GPK_TC_STATIC=0); the parity bar on the objective is 1e-5
+    # sqrt(K_ii), so a few leading digit bits are unused -- measured 6e-13 here (4e-14 with per-update row maxima);
+    # the parity bar on the objective is 1e-5
     assert num / den < 3e-12
 
 

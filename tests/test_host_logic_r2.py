@@ -32,7 +32,7 @@ def test_plane_store_packing_is_a_bijection_onto_a_dense_range():
     assert plane_prefix(66, 64) == 2 * 65 * 64 + 256
 
 
-def pick_slices(cond):  # mirror of csrc/potrf.cu::pick_slices (GPK_TC_SLICES unset)
+def pick_slices(cond):  # mirror of csrc/potrf.cu::pick_slices
     return 6 if 0 < cond <= 1e4 else 7
 
 
